@@ -30,6 +30,13 @@ Prints ONE JSON line (rank 0).  Keys beyond the base contract:
                crossing the boundary every vector step
   multi_rank_parity  (N > 1) the teacher-forced golden scenarios reproduced by the N ranks
                before timing ("ok" / error text)
+
+`--dump-outputs DIR` writes what the timed path computed in its last step as DIR/<name>.npy
+(rank 0), so that two builds run with the same arguments (same seeded inputs) can be compared
+output for output.
+
+The benchmark runs the library that `__graft_entry__.build()` left in the tree; it compiles
+nothing and writes nothing there.
 """
 
 import argparse
@@ -40,6 +47,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True      # the tree may be read-only
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -120,11 +128,8 @@ class Run:
         torch.cuda.set_device(self.local_rank)
         if self.world > 1:
             dist.init_process_group('nccl', device_id=torch.device('cuda', self.local_rank))
-        import __graft_entry__
-        if self.rank == 0:
-            __graft_entry__.build()
-        if self.world > 1:
-            dist.barrier()
+        from tonic_b200 import _lib
+        _lib.load()         # raises when the library has not been built
 
     def barrier(self):
         if self.world > 1:
@@ -197,6 +202,33 @@ def hbm_table(prof, bytes_per_launch, hbm_peak):
     return out
 
 
+DUMP_BYTES = 64 << 20       # --dump-outputs writes at most this much
+DUMP_ENVS = 1024            # environment columns of the PPO segment in the dump (fixed seeded sample)
+
+
+def dump_outputs(out_dir, tensors):
+    """Writes every tensor as out_dir/<name>.npy: float64 stays float64, everything else becomes
+    float32."""
+    import numpy as np
+    arrays = {}
+    for name, t in tensors.items():
+        a = t.detach().cpu().numpy()
+        arrays[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES, f'--dump-outputs: {total} bytes exceed the {DUMP_BYTES} byte limit'
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
+def model_outputs(agent, stats):
+    """What an update hands back: the model's state_dict (the reference's key names, as in a
+    checkpoint) and the per-minibatch statistics block the logger reads."""
+    out = {'model.' + k: v for k, v in agent.model.state_dict().items()}
+    out['update_stats'] = stats
+    return out
+
+
 # ----------------------------------------------------------------------------- PPO
 def build_ppo(envs_local, total_envs, seed=0):
     import torch
@@ -218,6 +250,21 @@ def build_ppo(envs_local, total_envs, seed=0):
     agent = tonic_b200.torch.agents.PPO(model=model, replay=replay)
     agent.initialize(env.observation_space, env.action_space, seed=seed)
     return agent, env, batch
+
+
+def ppo_outputs(agent, env):
+    """The last PPO iteration on a fixed seeded sample of environment columns: the segment it
+    collected with the values, returns and advantages of its update, and the observations the
+    next iteration starts from; then the updated model and the update's statistics."""
+    import numpy as np
+    import torch
+    n = env.workers
+    cols = np.sort(np.random.RandomState(0).choice(n, min(DUMP_ENVS, n), replace=False))
+    cols = torch.as_tensor(cols, device=env.observations.device)
+    out = {'segment.' + k: v.index_select(1, cols) for k, v in agent.replay.buffers.items()}
+    out['env.observations'] = env.observations.index_select(0, cols)
+    out.update(model_outputs(agent, agent._update_buffers[0]))
+    return out
 
 
 def multi_rank_parity(run):
@@ -279,6 +326,8 @@ def run_ppo(args):
     timed_iterations = dict(iterations)
     env_steps = args.steps * SEGMENT * total_envs
     value = env_steps / (elapsed_ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ppo_outputs(agent, env))
 
     if args.quick:
         if rank == 0:
@@ -518,9 +567,20 @@ def build_offpolicy(name, envs_local, total_envs, batch, seed=0):
     return agent, env
 
 
-def measure_offpolicy(run, name, steps, warmup, batch):
+def offpolicy_outputs(agent, env):
+    """The last vector step: the actions, what the environment returned for them (the transition
+    stored in the ring), the updated model and the update's statistics."""
+    out = {'actions': agent._staged_actions}
+    for k in ('observations', 'next_observations', 'rewards', 'resets', 'terminations'):
+        out['env.' + k] = getattr(env, k)
+    out.update(model_outputs(agent, agent._update_stats))
+    return out
+
+
+def measure_offpolicy(run, name, steps, warmup, batch, dump_dir=None):
     """Fills the device ring (untimed: collector only), then times `steps` vector steps, each
-    followed by the reference's update (50 iterations x batch)."""
+    followed by the reference's update (50 iterations x batch); `dump_dir`: writes the outputs
+    of the last timed step there."""
     import torch
     from tonic_b200 import _lib, config, kernels
     from tonic_b200.utils import logger
@@ -553,6 +613,8 @@ def measure_offpolicy(run, name, steps, warmup, batch):
     launches0 = _lib.launch_count() + graphs.replayed_launches
     ms = run.timed(vector_step, steps)
     launches = _lib.launch_count() + graphs.replayed_launches - launches0
+    if dump_dir and run.rank == 0:
+        dump_outputs(dump_dir, offpolicy_outputs(agent, env))
     update_ms = ms / steps - collect_ms      # device time added by the update to one vector step
     # instrumented pass (graphs off: per-launch events)
     config.graphs = False
@@ -610,7 +672,7 @@ def run_offpolicy(args):
     sampler = ClockSampler(run.local_rank)
     if run.rank == 0:
         sampler.start()
-    res = measure_offpolicy(run, name, args.steps, args.warmup, args.offpolicy_batch)
+    res = measure_offpolicy(run, name, args.steps, args.warmup, args.offpolicy_batch, args.dump_outputs)
     sampler.stop_flag = True
     if run.rank != 0:
         return
@@ -826,7 +888,13 @@ def main():
                              "(numpy-compatible MT19937 stream, bit-identical to the reference)")
     parser.add_argument('--quick', action='store_true',
                         help='timed region only (for runs under ncu): no e2e / cpu_baseline / profile pass')
+    parser.add_argument('--dump-outputs', metavar='DIR',
+                        help='write the outputs of the last timed step as DIR/<name>.npy')
     args = parser.parse_args()
+    if args.steps < 1:
+        parser.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        parser.error('--dump-outputs covers the GPU implementation only')
     if args.impl == 'reference':
         run_reference(args)
     else:
